@@ -2,6 +2,7 @@
 """bench.py — contrast-loss fwd+bwd throughput on synthetic Cityscapes-shaped batches (BASELINE.json metric).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl engine|reference] [--workload s1|s2]
+                    [--dump-outputs DIR]
 
 Workload s1 = BASELINE configs[1]: HRNet-W48 pixel-contrast (no bank), 1024x512 input -> 256x128 embedding,
 19 classes, batch 8 PER GPU (weak scaling; the no-bank loss has no cross-rank exchange, SURVEY §8e).
@@ -22,6 +23,7 @@ import time
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
 
+import numpy as np  # noqa: E402
 import torch  # noqa: E402
 
 S1 = dict(B=8, D=256, h=128, w=256, K=19, stride=4, block=32, T=0.1, bT=0.07, max_samples=1024, max_views=100)
@@ -466,6 +468,27 @@ def rotation_sets(cfg, bank):
     return max(2, min(8, -(-int(2.2 * L2_BYTES) // ws)))
 
 
+DUMP_GRAD_BYTES = 48 << 20          # keeps a --dump-outputs directory under 64 MB
+
+
+def output_sample(loss, grad):
+    """Host copy of one step's outputs for --dump-outputs.  The dense gradient (268 MB at the s1 shape) is cut down to a
+    fixed, seeded subset of its D channels at every pixel, so every sampled anchor column still shows up; a gradient that
+    fits the budget is kept whole.  grad_embed_channels lists the channels kept."""
+    B, D, h, w = grad.shape
+    keep = max(1, min(D, DUMP_GRAD_BYTES // (B * h * w * 4)))
+    ch = torch.arange(D) if keep == D else torch.randperm(D, generator=torch.Generator().manual_seed(0))[:keep].sort().values
+    g = grad.detach().index_select(1, ch.to(grad.device)).float().cpu()
+    return {"loss": np.float32(loss.item()), "grad_embed": g.numpy(),
+            "grad_embed_channels": ch.double().numpy()}
+
+
+def write_outputs(path, arrays):
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), a)
+
+
 class Workload:
     """One measured workload: R rotating input sets, one GraphedContrastStep per set (bank steps share the bank)."""
 
@@ -513,7 +536,16 @@ class Workload:
         if self.bank:
             self.mbank.enqueue(e.detach(), inp["target"], network_stride=self.cfg["net_stride"], pixel_update_freq=self.cfg["F"])
         loss.backward()
+        self.eager_out = (loss.detach(), e.grad)
         return loss
+
+    def step_outputs(self, i):
+        """What step i handed its caller: (loss, d loss/d embed).  Graph steps keep them in static buffers until the
+        same step object replays again."""
+        if self.steps:
+            st = self.steps[i % self.R]
+            return st.loss, st.grad
+        return self.eager_out
 
     def barrier(self):
         if self.world > 1:
@@ -526,8 +558,9 @@ class Workload:
             torch.distributed.all_reduce(t, op=torch.distributed.ReduceOp.MAX)
         return [float(v) for v in t.tolist()]
 
-    def time_loop(self, fn, steps, warmup, sampler=None):
+    def time_loop(self, fn, steps, warmup, sampler=None, after_timed=None):
         """K steps bracketed by barrier + synchronize, CUDA events on the launching stream, max over ranks.
+        after_timed(K - 1) runs once the timed steps have finished, before any further step.
         Returns (device ms per step, host enqueue ms per step, clock window description)."""
         for i in range(max(warmup, 3)):
             fn(i)
@@ -543,6 +576,8 @@ class Workload:
         ev[1].record()
         t_host = time.perf_counter() - t0               # host time to enqueue the K steps (no sync inside)
         self.barrier()
+        if after_timed is not None:
+            after_timed(steps - 1)
         window = "timed region"
         if sampler is not None:
             # nvidia-smi samples every 200 ms; a short timed region would see no sample, so the SAME loop keeps running
@@ -639,14 +674,18 @@ class Workload:
                 b.sync_shadow()
         return n
 
-    def measure(self, sampler=None, with_eager=False, with_e2e=True):
+    def measure(self, sampler=None, with_eager=False, with_e2e=True, keep_outputs=False):
+        """keep_outputs: self.outputs = a host copy (output_sample) of what the last timed step returned."""
         a = self.args
         out = {"workload": workload_config(self.cfg, self.bank)["workload"], "per_gpu_batch": self.cfg["B"],
                "rotation_sets": self.R, "working_set_mb": round(working_set_bytes(self.cfg, self.bank) / 1e6, 1)}
         fn, mode = (self.replay, "graph") if self.steps else (self.eager, "eager")
         if not self.steps:
             out["graph_error"] = self.graph_error or "disabled (--no-graph)"
-        ms, host, window = self.time_loop(fn, a.steps, a.warmup, sampler)
+
+        def keep(i):
+            self.outputs = output_sample(*self.step_outputs(i))
+        ms, host, window = self.time_loop(fn, a.steps, a.warmup, sampler, after_timed=keep if keep_outputs else None)
         out.update(mode=mode, ms_per_step=ms, value=self.world * self.cfg["B"] / (ms / 1e3), host_ms_per_step=host,
                    clock_window=window, kernels_per_step=self.kernels_per_step())
         if with_e2e:
@@ -703,7 +742,9 @@ def run_engine(args, cfg, bank, rank, world, dev):
     sampler = ClockSampler(dev.index)
     # ---- headline: the workload named on the command line (default s1 = BASELINE configs[1]), weak scaling ----
     head = Workload(args, args.workload, cfg, bank, rank, world, dev)
-    hm = head.measure(sampler=sampler, with_eager=True)
+    hm = head.measure(sampler=sampler, with_eager=True, keep_outputs=bool(args.dump_outputs))
+    if args.dump_outputs and rank == 0:
+        write_outputs(args.dump_outputs, head.outputs)
     A_live = int(head.steps[0].ws.plan[2].item()) if head.steps else 0
     timeline = head.graph_timeline() if not os.environ.get("PCL_BENCH_TINY") else None
     inp0 = head.inp[0]
@@ -885,8 +926,8 @@ def tensor_sweep_roofline(dev, peaks, A=16384, N=65536, iters=5):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=200)
-    ap.add_argument("--warmup", type=int, default=10)
+    ap.add_argument("--steps", type=int, default=None, help="timed steps [engine 200, reference 3]")
+    ap.add_argument("--warmup", type=int, default=None, help="warm-up steps [engine 10, reference 1]")
     ap.add_argument("--impl", default="engine", choices=["engine", "reference"])
     ap.add_argument("--workload", default="s1", choices=["s1", "s2", "s3"],
                     help="s1 = BASELINE configs[1] (headline), s2 = configs[2] (memory bank), s3 = configs[3] (171 classes)")
@@ -898,7 +939,19 @@ def main():
                     help="run GraphedContrastStep's launch sequence eagerly instead of as a captured CUDA graph")
     ap.add_argument("--precision", default="bf16", choices=["bf16", "fp32"],
                     help="InfoNCE sweeps: bf16 operands on tcgen05 tensor cores (default) or the exact fp32 SIMT sweep")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="engine arm: write the loss and d loss/d embed of the last timed step (rank 0) as DIR/<name>.npy; "
+                         "the gradient as a fixed channel sample when it exceeds 48 MB")
     args = ap.parse_args()
+    ref_arm = args.impl == "reference"
+    if args.steps is None:                           # the defaults are sized for the GPU arm
+        args.steps = 3 if ref_arm else 200
+    if args.warmup is None:
+        args.warmup = 1 if ref_arm else 10
+    if args.steps < 1:
+        raise SystemExit("--steps must be at least 1")
+    if ref_arm and args.dump_outputs:
+        raise SystemExit("--dump-outputs writes what the engine computed: use it with --impl engine")
     world = int(os.environ.get("WORLD_SIZE", "1"))
     rank = int(os.environ.get("RANK", "0"))
     local = int(os.environ.get("LOCAL_RANK", "0"))
@@ -912,9 +965,7 @@ def main():
         cfg.update(B=2, D=32, h=16, w=16, K=5, stride=2, block=8, max_samples=32, max_views=4)
         if bank:
             cfg.update(M=8, F=2, net_stride=2)
-    if args.impl == "reference":
-        if args.steps == 200 and args.warmup == 10:      # defaults are sized for the GPU arm
-            args.steps, args.warmup = 3, 1
+    if ref_arm:
         res = run_reference(args, cfg, bank, rank)
         if res is not None:
             print(json.dumps(res), flush=True)

@@ -1,6 +1,6 @@
-"""Generate golden vectors by running the UNMODIFIED reference (imported from /root/reference).
+"""Generate golden vectors by running the UNMODIFIED reference (located by oracle.ref_loader.reference_root()).
 
-Run in the build container only:  python tests/golden/make_golden.py
+Run where a reference tree is reachable:  python tests/golden/make_golden.py [aux | random_seeds]
 Writes tests/golden/*.npz.  The reference is fp32 PyTorch; every torch.randperm it draws is
 recorded so that the engine / the port can replay identical sample indices.
 """
@@ -167,12 +167,67 @@ def enqueue_case(name, *, B, D, h, w, K, img_stride, net_stride, M, Fq, steps, s
     print(f"{name}: steps={steps} final seg ptr={sp.tolist()} pix ptr={pp.tolist()}")
 
 
+def input_sums(*tensors):
+    """float64 sums of the inputs a case regenerates from contrastiveseg_b200.synth: a golden made from other data fails
+    loudly instead of comparing unrelated numbers."""
+    return np.array([t.double().sum().item() for t in tensors], dtype=np.float64)
+
+
+def random_seeds_case(name="random_seeds"):
+    """Reference outputs for tests/test_oracle_vs_reference.py: the loss on synth seeds 31-33 with and without the bank,
+    and five enqueue steps.  Only outputs and recorded permutations are stored; the tests regenerate the inputs."""
+    ref = load_reference()
+    out = {}
+    for seed in (31, 32, 33):
+        K, D = 6, 32
+        data = make_contrast_batch(B=3, D=D, h=20, w=24, num_classes=K, img_stride=2, block=6, seed=seed, boost=1.5)
+        predict = data["seg"].argmax(1)
+        for mem in (False, True):
+            cfg = DictConfiger(cfg_dict(0.1, 0.07, 50, 7))
+            key = f"s{seed}_mem{int(mem)}_"
+            sums = [data["embed"], data["target"], predict]
+            queue = None
+            if mem:
+                bank = make_bank(K, 15, D, seed)
+                queue = torch.cat((bank["segment_queue"], bank["pixel_queue"]), 1)
+                sums.append(queue)
+            rec = PermRecorder(torch.Generator().manual_seed(seed))
+            embed = data["embed"].clone().requires_grad_(True)
+            crit = (ref.mem if mem else ref.nomem).PixelContrastLoss(cfg)
+            with patched_randperm(rec):
+                loss = crit(embed, data["target"], predict, queue) if mem else crit(embed, data["target"], predict)
+            loss.backward()
+            out[key + "perm_flat"], out[key + "perm_lens"] = pack_perms(rec.draws)
+            out[key + "loss"] = np.float64(loss.item())
+            out[key + "grad_embed"] = embed.grad.numpy()
+            out[key + "input_sums"] = input_sums(*sums)
+    K, D, M, Fq = 5, 16, 6, 4
+    bank = make_bank(K, M, D, 3)
+    state = [bank[k].clone() for k in ("segment_queue", "segment_queue_ptr", "pixel_queue", "pixel_queue_ptr")]
+    me = types.SimpleNamespace(network_stride=2, memory_size=M, pixel_update_freq=Fq)
+    out["enq_input_sums"] = input_sums(*state)
+    for s in range(5):
+        data = make_contrast_batch(B=2, D=D, h=12, w=12, num_classes=K, img_stride=2, block=6, seed=50 + s)
+        rec = PermRecorder(torch.Generator().manual_seed(s))
+        with patched_randperm(rec):
+            ref.enqueue(me, data["embed"], data["target"], *state)
+        out[f"enq{s}_perm_flat"], out[f"enq{s}_perm_lens"] = pack_perms(rec.draws)
+        out[f"enq{s}_input_sums"] = input_sums(data["embed"], data["target"])
+        for k, t in zip(("sq", "sp", "pq", "pp"), state):
+            out[f"enq{s}_{k}"] = t.numpy().copy()
+    np.savez_compressed(os.path.join(HERE, name + ".npz"), **out)
+    print(f"{name}: " + " ".join(f"{k[:-4]}={v:.7f}" for k, v in out.items() if k.endswith("loss")))
+
+
 if __name__ == "__main__":
     only = sys.argv[1:]
     if only == ["aux"]:              # add the round-2 cases without touching the committed round-1 files
         torch.manual_seed(0)
         aux_wrapper_case("wrapper_aux_embed", with_embed=True)
         aux_wrapper_case("wrapper_aux_warmup_weighted", with_embed=False, weighted=True)
+        sys.exit(0)
+    if only == ["random_seeds"]:
+        random_seeds_case()
         sys.exit(0)
     torch.manual_seed(0)
     loss_case("nomem_small", B=2, D=32, h=24, w=24, K=5, stride=2, block=8, T=0.1, bT=0.07,
@@ -198,3 +253,4 @@ if __name__ == "__main__":
                  steps=6, seed=21)
     enqueue_case("enqueue_q6", B=2, D=32, h=16, w=16, K=5, img_stride=2, net_stride=4, M=9, Fq=4,
                  steps=4, seed=22)
+    random_seeds_case()

@@ -33,7 +33,7 @@ def test_reference_arm_bank_workload():
     assert d["impl"] == "reference" and "memory bank" in d["config"]["workload"]
 
 
-def _run_engine_on_emulator(monkeypatch, workload="s1"):
+def _run_engine_on_emulator(monkeypatch, workload="s1", dump=None):
     """bench.run_engine end to end on the CPU: the engine's kernels on the host-fiber emulator (tests/emu), CUDA events /
     pinned memory / graph capture stubbed, toy geometry.  Exercises everything between argument parsing and the JSON line."""
     import types
@@ -65,7 +65,7 @@ def _run_engine_on_emulator(monkeypatch, workload="s1"):
     orig_stage = bench.stage_timings
     monkeypatch.setattr(bench, "stage_timings", lambda *a, **k: orig_stage(*a, iters=2))        # the default 20 only averages
     args = types.SimpleNamespace(steps=4, warmup=3, precision="fp32", workload=workload, scaling="weak", no_graph=False,
-                                 no_cpu_baseline=False, gpus=1)
+                                 no_cpu_baseline=False, gpus=1, dump_outputs=dump)
     cfg = dict(bench.S1 if workload == "s1" else bench.S2)
     cfg.update(B=2, D=32, h=16, w=16, K=5, stride=2, block=8, max_samples=32, max_views=4)
     if workload != "s1":
@@ -96,6 +96,36 @@ def test_engine_arm_line_on_the_emulator(monkeypatch):
     bank = res["bank"]
     assert "error" not in bank and bank["mode"] == "graph" and bank["finite_loss"] and bank["kernels_per_step"] > r["kernels_per_step"]
     assert bank["value"] == 1 * 4 / 2e-3 and res["strong"] is None
+
+
+def test_engine_arm_dumps_the_last_timed_step(monkeypatch, tmp_path):
+    import numpy as np
+    import bench
+    monkeypatch.setenv("PCL_BENCH_HEADLINE_ONLY", "1")
+    monkeypatch.setattr(bench, "DUMP_GRAD_BYTES", 8 * 2 * 16 * 16 * 4)     # 8 of the toy gradient's 32 channels
+    seen, replays = [], []
+    orig_sample, orig_replay = bench.output_sample, bench.Workload.replay
+
+    def spy(loss, grad):
+        seen.append((loss.item(), grad.clone()))
+        return orig_sample(loss, grad)
+
+    def replay(self, i):
+        loss = orig_replay(self, i)
+        replays.append(loss.item())
+        return loss
+    monkeypatch.setattr(bench, "output_sample", spy)
+    monkeypatch.setattr(bench.Workload, "replay", replay)
+    _run_engine_on_emulator(monkeypatch, dump=str(tmp_path))
+    assert sorted(os.listdir(tmp_path)) == ["grad_embed.npy", "grad_embed_channels.npy", "loss.npy"]
+    loss, grad, ch = (np.load(os.path.join(tmp_path, n + ".npy")) for n in ("loss", "grad_embed", "grad_embed_channels"))
+    assert len(seen) == 1 and loss.dtype == grad.dtype == np.float32 and ch.dtype == np.float64
+    # 3 warm-up + 4 timed replays: the dump is the 7th, although the run replays the step again afterwards
+    assert len(replays) > 7 and replays[6] != replays[-1]
+    assert loss.shape == () and float(loss) == seen[0][0] == replays[6]
+    idx = ch.astype(np.int64)
+    assert grad.shape == (2, 8, 16, 16) and list(idx) == sorted(set(idx)) and 0 <= idx[0] and idx[-1] < 32
+    assert np.array_equal(grad, seen[0][1][:, idx].numpy()) and np.count_nonzero(grad) > 0
 
 
 def test_engine_arm_bank_workload_as_headline(monkeypatch):

@@ -109,3 +109,9 @@ def device_step_seed(seed: int, step_counter: int) -> int:
 def device_rank(step_seed: int, image: int, cls: int, num_classes: int, easy: bool, j: int, n: int) -> int:
     """Rank (within the hard or easy pixel list of (image, cls), ascending pixel order) of the j-th sampled view."""
     return keyed_perm(j, n, mix64(step_seed ^ (((image * num_classes + cls) << 1) | (1 if easy else 0))))
+
+
+def device_bank_rank(enqueue_seed: int, slot: int, j: int, n: int) -> int:
+    """Pixel column of the j-th row that the bank enqueue (csrc/pcl_bank.cu k_bank_rows) takes from the n pixels of
+    slot = image * num_classes + class, for the seed the packet kernel receives (bank.enqueue_seed(seed) + call counter)."""
+    return keyed_perm(j, n, mix64((enqueue_seed ^ (0xB5 << 56) ^ slot) & _M64))

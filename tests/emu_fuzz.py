@@ -146,7 +146,7 @@ def fuzz_segce(seed: int, n: int):
     rng = random.Random(seed)
     bad = []
     for it in range(n):
-        B, K, h, w = rng.randint(1, 3), rng.randint(2, 21), rng.randint(1, 20), rng.randint(1, 24)
+        B, K, h, w = rng.randint(1, 3), rng.randint(2, 60), rng.randint(1, 20), rng.randint(1, 24)
         H, W, weighted, ign = rng.randint(1, 60), rng.randint(1, 60), rng.random() < 0.5, rng.choice([-1, 255, 0])
         g = torch.Generator().manual_seed(rng.randint(0, 10 ** 6))
         seg = torch.randn(B, K, h, w, generator=g) * 2

@@ -1,7 +1,7 @@
 """CPU execution of the engine's REAL kernel sources (tests/emu: the .cu files compiled for host fibers; the tensor path
 against a functional model of mbarrier / TMA / tcgen05): the GPU tests of test_gpu_parity.py / test_gpu_topk.py /
 test_gpu_zpending.py are re-run here with DEV = "cpu", through the same Python layer and the same C ABI (all but the
-full-size ones).  This covers the kernel logic (indices,
+full-size ones), and the small cases of test_gpu_edges.py / test_gpu_zpending_edges.py.  This covers the kernel logic (indices,
 barriers, reductions, selection, sampling, bank update, top-k select, graph rank draw) on machines without a GPU; it
 proves nothing about the hardware build (that is what `-m gpu` is for) and floating point differs from the GPU in the
 last bits (no FMA contraction), which the parity tolerances absorb.  TEST INFRASTRUCTURE: the product never loads the
@@ -14,12 +14,14 @@ import emu_harness
 import test_gpu_parity as G
 import test_gpu_zpending as PD
 import test_gpu_topk as TK
+import test_gpu_edges as GE
+import test_gpu_zpending_edges as ZE
 
 
 @pytest.fixture
 def emu(monkeypatch):
     lib = emu_harness.use_emulation(monkeypatch)
-    for m in (G, TK, PD):
+    for m in (G, TK, PD, GE, ZE):
         monkeypatch.setattr(m, "DEV", "cpu")
     monkeypatch.setattr(torch.cuda, "synchronize", lambda *a, **k: None)
     # the GPU tests rely on `.to(DEV)` producing a NEW tensor (host -> device copy); `.to("cpu")` would alias the source
@@ -304,3 +306,46 @@ def test_device_sampler_equals_its_host_model(emu):
                 want += [(b, c, hard[rng.device_rank(seed, b, c, K, False, j, len(hard))]) for j in range(kh)]
                 want += [(b, c, easy[rng.device_rank(seed, b, c, K, True, j, len(easy))]) for j in range(ke)]
         assert got == sorted(want)
+
+
+EDGES = (
+    [_case(GE.test_tc_self_mode_at_row_tile_edges, A=a) for a in (2, 129, 257)] +
+    [_case(GE.test_tc_explicit_mode_at_tile_edges, A=a, N=n) for a, n in ((1, 1), (128, 255), (129, 257), (129, 513))] +
+    [_case(GE.test_tc_class_blocks_on_half_tile_boundaries, blocks=0, sorted_cols=s) for s in (True, False)] +
+    [_case(GE.test_tc_nan_safe_row_without_positive)] +
+    [_case(GE.test_tc_bank_class_blocks_at_tile_edges, M=m) for m in (63, 128)] +
+    [_case(GE.test_segce_class_chunks, K=k, weighted=wt, ign=ig) for k, wt, ig in ((25, False, -1), (33, True, 255),
+                                                                                 (59, True, -1), (171, False, 255))]
+)
+
+
+@pytest.mark.parametrize("fn,kw", EDGES)
+def test_tile_and_chunk_edges_on_emulation(emu, fn, kw):
+    """The small cases of test_gpu_edges.py: tcgen05 sweeps at 128/256 tile edges, class blocks on half-tile boundaries
+    (sorted and shuffled columns), non-zero contrast pad rows, nan_safe, and seg-CE over several class chunks."""
+    fn(**kw)
+
+
+def _uncaptured(monkeypatch):
+    from contrastiveseg_b200 import graph_step
+    monkeypatch.setattr(graph_step.GraphedContrastStep, "_capture", lambda self, warmup: None)
+    monkeypatch.setattr(graph_step.GraphedContrastStep, "_fork_zero_fill", lambda self: self._side_branch(0))
+    monkeypatch.setattr(graph_step.GraphedContrastStep, "_join_zero_fill", lambda self: None)
+
+
+@pytest.mark.parametrize("A,TC,V,ms,mv", [(4, 2, 2, 1024, 2), (129, 3, 43, 130, 43)])
+def test_fused_step_at_exact_anchor_counts_on_emulation(emu, monkeypatch, A, TC, V, ms, mv):
+    """The fused step's launch sequence (uncaptured) at exact anchor counts against the host model and float64."""
+    _uncaptured(monkeypatch)
+    ZE.test_fused_step_at_exact_anchor_counts(A, TC, V, ms, mv)
+
+
+def test_fused_step_anchor_count_changes_on_emulation(emu, monkeypatch):
+    """A = 1024 -> 129 -> 4 -> 1024 through one step object with sparse_reset: no row of a larger replay leaks."""
+    _uncaptured(monkeypatch)
+    ZE.test_fused_step_anchor_count_changes_between_replays(True)
+
+
+def test_device_bank_rank_on_emulation(emu):
+    """The host model of the enqueue draw equals k_bank_rows' own draw (packets bit for bit)."""
+    ZE.test_device_bank_rank_is_the_packet_kernels_draw()
